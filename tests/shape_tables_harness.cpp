@@ -26,6 +26,12 @@ void sth_cube(void *p, float *ub2, float *lb2, float *wide2 /* 4 levels, concate
   std::memcpy(lb2, t->cube_lb2.data(), nc * sizeof(float));
   for (int lv = 0; lv < 4; lv++) std::memcpy(wide2 + lv * nc, t->cube_wide2[lv].data(), nc * sizeof(float));
 }
+void sth_frame(void *p, double *out) {   // volume, com[3], inertia[3], quat_principal[4]
+  auto *t = static_cast<shgpu::ShapeTables *>(p);
+  out[0] = t->volume;
+  for (int d = 0; d < 3; d++) { out[1 + d] = t->com[d]; out[4 + d] = t->inertia[d]; }
+  for (int d = 0; d < 4; d++) out[7 + d] = t->quat_principal[d];
+}
 void sth_nodes(void *p, double *pts, double *nds) {
   auto *t = static_cast<shgpu::ShapeTables *>(p);
   for (int k = 0; k < t->nq; k++) for (int d = 0; d < 3; d++) { pts[3 * k + d] = t->node_p[d][k]; nds[3 * k + d] = t->node_n[d][k]; }
