@@ -128,6 +128,24 @@ int sh_get_energy(const sh_ctx *h, double *ke_trans, double *ke_rot, double *e_c
  * sum_pairs (x_i - x_j) (x) F_i with pairs that involve a ghost counted half; pressure tensor = (kinetic + virial summed
  * over the ranks) / box volume.  Wall forces are not included. */
 int sh_get_stress(const sh_ctx *h, double virial[9], double kinetic[9]);
+/* compute stress/atom, pe/atom, contact/atom: per-atom quantities of the first n owned atoms (sh_get_atoms order, row i of
+ * each output), from the forces of the last sh_compute_forces / sh_run step (the state sh_get_stress reads).  Sums over
+ * every pair (i, j) of atom i:
+ *   virial   (n x 9, row-major 3a+b)  mode 0 (LAMMPS compute stress/atom): W_i = sum_j 1/2 (x_i - x_j)_a F_ij,b with the
+ *            centre-of-mass separation (periodic / Lees-Edwards image) of sh_get_stress and F_ij the force on i;
+ *            mode 1 (contact branch vectors, Love-Weber per-particle stress): W_i = sum_j (x_i - x_c)_a F_ij,b with x_c the
+ *            pair's overlap centroid (sh_get_pairs), so a contact's moment goes to the particle whose surface carries it;
+ *            a pair with V <= 0 contributes nothing.  In both modes the sum over all owned atoms (and ranks) equals
+ *            sh_get_stress's virial up to summation order.  Walls contribute no virial.
+ *   kinetic  (n x 9)  m v_a v_b; sums to sh_get_stress's kinetic.
+ *   energy   (n)      1/2 sum_j E_ij + wall energy of i; sums to sh_get_energy's e_contact.
+ *   contacts (n)      pairs of i with V > 0 (wall contacts are not counted).
+ * NULL outputs are skipped; n out of [0, owned atoms] or a mode other than 0 / 1 fails.  Without valid forces the pair
+ * and wall parts are zero.  Fixed-order sums: two calls on the same state are bitwise equal, and the call leaves the
+ * trajectory untouched.  In-library decomposition: collective (every rank calls it); with newton on the halves held by
+ * ghost rows are returned to their owners. */
+int sh_get_atom_stress(const sh_ctx *h, int64_t n, int mode, double *virial, double *kinetic, double *energy,
+                       int *contacts);
 int sh_get_counters(const sh_ctx *h, int64_t *pair_evals, int64_t *nodes_transformed,
                     int64_t *nodes_evaluated, int64_t *nodes_inside, int64_t *neighbor_builds,
                     int64_t *kernel_launches);

@@ -129,6 +129,15 @@ class ShGpu:
         self._ck(self.L.sh_get_stress(self.h, _p(w), _p(k)))
         return dict(virial=w.reshape(3, 3), kinetic=k.reshape(3, 3))
 
+    def get_atom_stress(self, mode=0):
+        """Per-atom virial (n,3,3), kinetic (n,3,3), energy (n,) and contacts (n,) of the owned atoms (include/shgpu.h
+        sh_get_atom_stress).  mode 0: centre-to-centre halves (LAMMPS compute stress/atom); 1: contact branch vectors.
+        Collective in a decomposed run: every rank calls it; n = nlocal."""
+        n = self.dd_info()["nlocal"] if self.dd else self.n
+        w, k, e, c = np.zeros((n, 3, 3)), np.zeros((n, 3, 3)), np.zeros(n), np.zeros(n, dtype=np.int32)
+        self._ck(self.L.sh_get_atom_stress(self.h, C.c_int64(n), int(mode), _p(w), _p(k), _p(e), _p(c, c_ip)))
+        return dict(virial=w, kinetic=k, energy=e, contacts=c)
+
     def add_wall(self, point, normal, k, exponent):
         p, nn = _d(point), _d(normal)
         self._ck(self.L.sh_add_wall(self.h, _p(p), _p(nn), C.c_double(k), C.c_double(exponent)))

@@ -22,6 +22,7 @@
 #include "pair_split_kernels.cuh"
 #include "shape_tables.h"
 #include "step_kernels.cuh"
+#include "atom_stress_kernels.cuh"
 
 using namespace shgpu;
 
@@ -147,6 +148,9 @@ struct sh_ctx {
   double sec_pair = 0, sec_neigh = 0, sec_comm = 0, sec_other = 0, sec_run_last = 0, sec_run_total = 0;
   cudaEvent_t run_e0 = nullptr, run_e1 = nullptr;
   int64_t pair_launches = 0;
+  // sh_get_atom_stress: per-atom outputs, entry -> pair map, newton-on ghost records (allocated by its first call)
+  DevBuf<double> as_vir, as_kin, as_en, as_send, as_recv;
+  DevBuf<int> as_cnt, as_epair;
   // tuning
   int tune_threads = 0, tune_ctas_per_sm = 0, tune_variant = 0, tune_cull_wpb = 0, tune_cull_lpp = 0;
 };
@@ -860,6 +864,7 @@ int sh_destroy(sh_ctx *h) {
                        &h->cnt_half, &h->nbr_off, &h->half_off, &h->nbr_j, &h->pair_i, &h->pair_j, &h->pair_eij, &h->pair_eji, &h->pair_img, &h->scalars};
   for (auto *b : ib) b->release();
   h->counters.release();
+  h->as_vir.release(); h->as_kin.release(); h->as_en.release(); h->as_send.release(); h->as_recv.release(); h->as_cnt.release(); h->as_epair.release();
   for (auto &e : h->ev) cudaEventDestroy(e);
   for (auto &e : h->ev2) cudaEventDestroy(e);
   h->pool.release(); h->pool_flag.release(); h->pool_base.release(); h->pool_cap.release(); h->split_sc.release(); h->eval_plan.release(); h->slow_list.release();
@@ -1536,6 +1541,63 @@ int sh_get_stress(const sh_ctx *hc, double virial[9], double kinetic[9]) try {
   if (n > 0) for (int b = 0; b < nb_atoms; b++) for (int k = 0; k < 9; k++) K[k] += part[(size_t)9 * b + k];
   if (np > 0) for (int b = 0; b < nb_pairs; b++) for (int k = 0; k < 9; k++) W[k] += part[(size_t)9 * (nb_atoms + b) + k];
   for (int k = 0; k < 9; k++) { if (virial) virial[k] = W[k]; if (kinetic) kinetic[k] = K[k]; }
+  return 0;
+} catch (...) { return -99; }   // no C++ exception crosses the C ABI (out of memory / internal error)
+
+// per-atom virial / kinetic tensor / contact energy / contact count of the owned atoms (compute stress/atom, pe/atom,
+// contact/atom).  Fixed-order sums over the CSR rows, no FP atomics; nothing here is part of a step.  Newton on in the
+// in-library decomposition: the ghost rows' halves go back to their owners through the reverse plan (collective).
+int sh_get_atom_stress(const sh_ctx *hc, int64_t n, int mode, double *virial, double *kinetic, double *energy, int *contacts) try {
+  sh_ctx *h = const_cast<sh_ctx *>(hc);
+  const int nown = (int)(h->n - h->nghost);
+  if (n < 0 || n > nown) return fail(h, "get_atom_stress: n out of range");
+  if (mode != 0 && mode != 1) return fail(h, "get_atom_stress: mode must be 0 (centre-to-centre) or 1 (contact centroid)");
+  CU(cudaSetDevice(h->device));
+  int rc = prepare(h);
+  if (rc) return rc;
+  DdCtx &D = h->dd;
+  const bool newton_dd = D.on && D.newton && D.borders_ok && (h->nghost > 0 || D.nsend > 0);
+  const bool pairs = h->forces_valid && h->list_valid && h->npairs > 0;
+  const int nall = newton_dd ? (int)h->n : nown;
+  const int nrows = pairs ? std::min(h->nrows, nall) : 0;
+  try {
+    h->as_vir.ensure((size_t)9 * std::max(nown, 1)); h->as_kin.ensure((size_t)9 * std::max(nown, 1));
+    h->as_en.ensure(std::max(nown, 1)); h->as_cnt.ensure(std::max(nown, 1));
+    if (pairs) h->as_epair.ensure((size_t)h->nentries + 1);
+    if (newton_dd) { h->as_send.ensure((size_t)11 * std::max<int64_t>(h->nghost, 1)); h->as_recv.ensure((size_t)11 * std::max(D.nsend, 1)); }
+  } catch (std::string &e) { return fail(h, e); }
+  if (pairs) {
+    CU(cudaMemsetAsync(h->as_epair.p, 0xff, (size_t)h->nentries * sizeof(int), h->stream));
+    atom_stress_entry_pair_kernel<<<cdiv(h->npairs, 256), 256, 0, h->stream>>>(h->npairs, h->pair_eij.p, h->pair_eji.p, h->as_epair.p);
+    h->kernel_launches++;
+  }
+  if (nall > 0) {
+    AtomStressArgs S;
+    S.A = view(h); S.shapes = h->d_shapes.p; S.nall = nall; S.nrows = nrows; S.mode = mode;
+    S.nbr_off = h->nbr_off.p; S.epair = h->as_epair.p; S.pair_i = h->pair_i.p; S.pair_j = h->pair_j.p; S.pair_img = h->pair_img.p;
+    S.pres = h->pres.p; S.pres_stride = h->pres_stride;
+    for (int d = 0; d < 3; d++) S.L[d] = h->hi[d] - h->lo[d];
+    S.ewall = h->forces_valid && h->walls.n > 0 ? h->ewall.p : nullptr;
+    S.vir = h->as_vir.p; S.kin = h->as_kin.p; S.en = h->as_en.p; S.cnt = h->as_cnt.p; S.ghost_rec = h->as_send.p;
+    atom_stress_row_kernel<<<cdiv(nall, 128), 128, 0, h->stream>>>(S);
+    h->kernel_launches++;
+  }
+  if (newton_dd) {
+    if ((rc = dd_sendrecv(h, D.nbr_rank, h->as_send.p, D.recv_cnt, h->as_recv.p, D.send_cnt, 11))) return rc;
+    if (D.nsend > 0 && nown > 0) {
+      atom_stress_add_returned_kernel<<<cdiv(nown, 256), 256, 0, h->stream>>>(nown, D.rev_off.p, D.rev_k.p, h->as_recv.p, h->as_vir.p,
+                                                                            h->as_en.p, h->as_cnt.p);
+      h->kernel_launches++;
+    }
+  }
+  CU(cudaGetLastError());
+  CU(cudaStreamSynchronize(h->stream));
+  if (n > 0) {
+    if (virial) CU(cudaMemcpy(virial, h->as_vir.p, (size_t)9 * n * sizeof(double), cudaMemcpyDeviceToHost));
+    if (kinetic) CU(cudaMemcpy(kinetic, h->as_kin.p, (size_t)9 * n * sizeof(double), cudaMemcpyDeviceToHost));
+    if (energy) CU(cudaMemcpy(energy, h->as_en.p, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost));
+    if (contacts) CU(cudaMemcpy(contacts, h->as_cnt.p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost));
+  }
   return 0;
 } catch (...) { return -99; }   // no C++ exception crosses the C ABI (out of memory / internal error)
 

@@ -12,8 +12,15 @@
 // vx vy vz ; velocity <id> set ... ; pair_style spherharm ; pair_coeff i j k exponent [gamma_n gamma_t mu] ; fix <id> <grp>
 // nve/sh | wall/spherharm <xplane|yplane|zplane> <pos> <k> <exponent> [hi] | gravity <g> vector x y z |
 // viscous <gamma> ; neighbor <skin> bin ; neigh_modify every N [check yes|no] ; timestep ; thermo N ;
-// dump <id> <grp> custom N <file> ... ; run N ; write_restart <file> ; read_restart <file> ; print "..." ;
+// compute <id> all stress/atom NULL [ke] [pair] [virial] [branch center|centroid] | pe/atom | contact/atom ;
+// dump <id> all custom N <file> <columns> (id type x y z vx vy vz qw qx qy qz fx fy fz tqx tqy tqz angmomx angmomy angmomz
+// c_ID c_ID[k]) ; run N ; write_restart <file> ; read_restart <file> ; print "..." ;
 // fix <id> <grp> deform N xy erate <rate> remap v   (Lees-Edwards shear: flow x, gradient y)
+//
+// compute stress/atom gives LAMMPS's 6-vector -(K + W) (xx yy zz xy xz yz; K = m v v, W the per-atom pair virial of
+// sh_get_atom_stress) in stress x volume units.  `branch centroid` (a shlmp extension) takes W from the contact branch
+// vectors (particle centre to overlap centroid, the granular-mechanics per-particle stress) instead of the LAMMPS
+// centre-to-centre halves.
 //
 // shlmp -gpus N: N ranks = N threads of this process, one GPU each, every rank interprets the script (as MPI ranks do in
 // LAMMPS); the domain decomposition, ghost exchange and migration run inside libshgpu (sh_dd_*, NCCL); rank 0 prints
@@ -93,7 +100,23 @@ void read_shape_file(const std::string &fn, int lmax, std::vector<double> &a, st
   }
 }
 
-struct Dump { std::string file; int every = 0; };
+// per-atom computes (compute stress/atom, pe/atom, contact/atom), all evaluated by sh_get_atom_stress
+struct Compute {
+  std::string id;
+  enum Style { STRESS, PE, CONTACT } style = STRESS;
+  bool ke = true, pair = true;
+  int mode = 0;                                   // sh_get_atom_stress mode: 0 centre-to-centre, 1 contact centroid
+  int ncols() const { return style == STRESS ? 6 : 0; }   // 0 = per-atom scalar
+};
+
+// one dump custom column: an atom attribute, or column `col` of compute `ci` (-1 = its scalar)
+struct DumpCol {
+  enum Kind { ID, TYPE, X, V, Q, F, TQ, L, COMP } kind = ID;
+  int comp = 0, ci = -1, col = -1;
+};
+const char *kDefaultDumpCols = "id type x y z qw qx qy qz vx vy vz";
+
+struct Dump { std::string file, header; int every = 0; std::vector<DumpCol> cols; };
 
 // the ranks of one shlmp job (threads): a reusable barrier and per-rank slots for gathers / reductions
 struct Team {
@@ -101,7 +124,7 @@ struct Team {
   char uid[128] = {0};
   std::mutex m; std::condition_variable cv; int waiting = 0; long generation = 0;
   bool failed = false;
-  struct Part { std::vector<int64_t> tag; std::vector<double> x, v, quat; double e[3] = {0, 0, 0}; };
+  struct Part { std::vector<int64_t> tag; std::vector<double> x, v, quat, extra; double e[3] = {0, 0, 0}; };
   std::vector<Part> part;
   void barrier() {
     std::unique_lock<std::mutex> lk(m);
@@ -128,6 +151,7 @@ struct Shlmp {
   int every = 1, check = 1, thermo = 0;
   int64_t step = 0;
   std::vector<Dump> dumps;
+  std::vector<Compute> computes;
   std::string restart_file;
   int rank = 0, nranks = 1;
   Team *team = nullptr;
@@ -136,6 +160,13 @@ struct Shlmp {
   std::unordered_map<int64_t, int> type_of_tag;
   // this rank's owned atoms as last pulled from the device
   std::vector<int64_t> ltag; std::vector<double> lx, lv, lq;
+  // per-atom values that the dumps of the current step need beyond x / v / quat, in avec order, `nextra` per atom:
+  // f (3), torque (3), angmom (3) when wanted, then the columns of every wanted compute (extra_off[ci], -1 = not pulled)
+  std::vector<double> extra;
+  int nextra = 0;
+  std::vector<int> extra_off;
+  enum { EX_F = 0, EX_TQ = 1, EX_L = 2 };
+  int ex_off[3] = {-1, -1, -1};
 
   void ck(int rc) { if (rc != 0) error_all(FLERR, sh_last_error(h)); }
   bool master() const { return rank == 0; }
@@ -190,12 +221,70 @@ struct Shlmp {
     for (size_t i = 0; i < avec.nlocal(); i++) type_of_tag[avec.tag[i]] = avec.type[i];
     initialised = true;
   }
+  // which per-atom values beyond x / v / quat the given dumps need: fills ex_off / extra_off / nextra
+  void plan_extra(const std::vector<const Dump *> &due) {
+    bool want[3] = {false, false, false};
+    std::vector<bool> wc(computes.size(), false);
+    for (auto *d : due)
+      for (auto &c : d->cols) {
+        if (c.kind == DumpCol::F) want[EX_F] = true;
+        else if (c.kind == DumpCol::TQ) want[EX_TQ] = true;
+        else if (c.kind == DumpCol::L) want[EX_L] = true;
+        else if (c.kind == DumpCol::COMP) wc[c.ci] = true;
+      }
+    nextra = 0;
+    for (int k = 0; k < 3; k++) { ex_off[k] = want[k] ? nextra : -1; nextra += want[k] ? 3 : 0; }
+    extra_off.assign(computes.size(), -1);
+    for (size_t ci = 0; ci < computes.size(); ci++)
+      if (wc[ci]) { extra_off[ci] = nextra; nextra += std::max(1, computes[ci].ncols()); }
+  }
+  // the planned extra values of this rank's first nl owned atoms (device order), nextra per atom.  sh_get_atom_stress is
+  // collective in a decomposed run: every rank gets here with the same plan.
+  std::vector<double> local_extra(int64_t nl) {
+    std::vector<double> out((size_t)nl * nextra);
+    if (nextra == 0) return out;
+    std::vector<double> a3[3];
+    for (int k = 0; k < 3; k++) if (ex_off[k] >= 0) a3[k].resize(3 * nl);
+    if (nl && (ex_off[EX_F] >= 0 || ex_off[EX_TQ] >= 0 || ex_off[EX_L] >= 0))
+      ck(sh_get_atoms(h, nl, nullptr, nullptr, nullptr, ex_off[EX_L] >= 0 ? a3[EX_L].data() : nullptr,
+                      ex_off[EX_F] >= 0 ? a3[EX_F].data() : nullptr, ex_off[EX_TQ] >= 0 ? a3[EX_TQ].data() : nullptr));
+    for (int k = 0; k < 3; k++)
+      if (ex_off[k] >= 0) for (int64_t i = 0; i < nl; i++) for (int d = 0; d < 3; d++) out[(size_t)nextra * i + ex_off[k] + d] = a3[k][3 * i + d];
+    for (int mode = 0; mode < 2; mode++) {
+      bool any = false;
+      for (size_t ci = 0; ci < computes.size(); ci++) any = any || (extra_off[ci] >= 0 && computes[ci].mode == mode);
+      if (!any) continue;
+      std::vector<double> W((size_t)9 * nl), K((size_t)9 * nl), E(nl);
+      std::vector<int> C(nl);
+      ck(sh_get_atom_stress(h, nl, mode, W.data(), K.data(), E.data(), C.data()));
+      for (size_t ci = 0; ci < computes.size(); ci++) {
+        const Compute &c = computes[ci];
+        if (extra_off[ci] < 0 || c.mode != mode) continue;
+        for (int64_t i = 0; i < nl; i++) {
+          double *o = &out[(size_t)nextra * i + extra_off[ci]];
+          if (c.style == Compute::PE) o[0] = E[i];
+          else if (c.style == Compute::CONTACT) o[0] = (double)C[i];
+          else {
+            static const int comp[6] = {0, 4, 8, 1, 2, 5};   // xx yy zz xy xz yz
+            for (int k = 0; k < 6; k++) {
+              double s = 0.0;
+              if (c.ke) s += K[9 * i + comp[k]];
+              if (c.pair) s += W[9 * i + comp[k]];
+              o[k] = -s;
+            }
+          }
+        }
+      }
+    }
+    return out;
+  }
   // device -> host staging (dump / thermo).  Decomposed runs: every rank pulls its owned atoms, rank 0 merges them by tag
-  // into the script-order arrays of avec.
+  // into the script-order arrays of avec (and `extra`, as planned by plan_extra).
   void pull_state() {
     if (!decomposed) {
       const int64_t n = (int64_t)avec.nlocal();
       if (n) ck(sh_get_atoms(h, n, avec.x.data(), avec.v.data(), avec.quat.data(), avec.angmom.data(), nullptr, nullptr));
+      extra = local_extra(n);
       return;
     }
     int64_t nl = 0, ng = 0;
@@ -206,15 +295,18 @@ struct Shlmp {
     Team::Part mine;
     mine.tag.assign(tg.begin(), tg.begin() + nl); mine.x.assign(x.begin(), x.begin() + 3 * nl); mine.v.assign(v.begin(), v.begin() + 3 * nl);
     mine.quat.assign(q.begin(), q.begin() + 4 * nl);
+    mine.extra = local_extra(nl);
     if (team) { team->part[rank] = std::move(mine); team->barrier(); }
     if (master()) {
       std::unordered_map<int64_t, size_t> where;
       for (size_t i = 0; i < avec.nlocal(); i++) where[avec.tag[i]] = i;
+      extra.assign(avec.nlocal() * nextra, 0.0);
       auto merge = [&](const Team::Part &p) {
         for (size_t k = 0; k < p.tag.size(); k++) {
           const size_t i = where.at(p.tag[k]);
           for (int d = 0; d < 3; d++) { avec.x[3 * i + d] = p.x[3 * k + d]; avec.v[3 * i + d] = p.v[3 * k + d]; }
           for (int d = 0; d < 4; d++) avec.quat[4 * i + d] = p.quat[4 * k + d];
+          for (int d = 0; d < nextra; d++) extra[(size_t)nextra * i + d] = p.extra[(size_t)nextra * k + d];
         }
       };
       if (team) for (auto &p : team->part) merge(p); else merge(mine);
@@ -236,19 +328,43 @@ struct Shlmp {
     fflush(stdout);
   }
   void write_dumps(bool force) {
-    for (auto &d : dumps) {
-      if (!force && (d.every <= 0 || step % d.every)) continue;
-      pull_state();
-      if (!master()) continue;
+    std::vector<const Dump *> due;
+    for (auto &d : dumps) if (force || (d.every > 0 && step % d.every == 0)) due.push_back(&d);
+    if (due.empty()) return;
+    plan_extra(due);
+    pull_state();
+    if (!master()) return;
+    std::string line;
+    char buf[64];
+    for (auto *dp : due) {
+      const Dump &d = *dp;
       FILE *f = fopen(d.file.c_str(), step == 0 || force ? (step == 0 ? "w" : "a") : "a");
       if (!f) error_all(FLERR, "Cannot open dump file " + d.file);
       fprintf(f, "ITEM: TIMESTEP\n%lld\nITEM: NUMBER OF ATOMS\n%zu\nITEM: BOX BOUNDS\n", (long long)step, avec.nlocal());
       for (int k = 0; k < 3; k++) fprintf(f, "%.17g %.17g\n", lo[k], hi[k]);
-      fprintf(f, "ITEM: ATOMS id type x y z qw qx qy qz vx vy vz\n");
-      for (size_t i = 0; i < avec.nlocal(); i++)
-        fprintf(f, "%lld %d %.17g %.17g %.17g %.17g %.17g %.17g %.17g %.17g %.17g %.17g\n", (long long)avec.tag[i], avec.type[i],
-                avec.x[3 * i], avec.x[3 * i + 1], avec.x[3 * i + 2], avec.quat[4 * i], avec.quat[4 * i + 1], avec.quat[4 * i + 2],
-                avec.quat[4 * i + 3], avec.v[3 * i], avec.v[3 * i + 1], avec.v[3 * i + 2]);
+      fprintf(f, "ITEM: ATOMS %s\n", d.header.c_str());
+      for (size_t i = 0; i < avec.nlocal(); i++) {
+        line.clear();
+        for (size_t k = 0; k < d.cols.size(); k++) {
+          const DumpCol &c = d.cols[k];
+          const double *ex = extra.data() + (size_t)nextra * i;
+          switch (c.kind) {
+            case DumpCol::ID: snprintf(buf, sizeof buf, "%lld", (long long)avec.tag[i]); break;
+            case DumpCol::TYPE: snprintf(buf, sizeof buf, "%d", avec.type[i]); break;
+            case DumpCol::X: snprintf(buf, sizeof buf, "%.17g", avec.x[3 * i + c.comp]); break;
+            case DumpCol::V: snprintf(buf, sizeof buf, "%.17g", avec.v[3 * i + c.comp]); break;
+            case DumpCol::Q: snprintf(buf, sizeof buf, "%.17g", avec.quat[4 * i + c.comp]); break;
+            case DumpCol::F: snprintf(buf, sizeof buf, "%.17g", ex[ex_off[EX_F] + c.comp]); break;
+            case DumpCol::TQ: snprintf(buf, sizeof buf, "%.17g", ex[ex_off[EX_TQ] + c.comp]); break;
+            case DumpCol::L: snprintf(buf, sizeof buf, "%.17g", ex[ex_off[EX_L] + c.comp]); break;
+            case DumpCol::COMP: snprintf(buf, sizeof buf, "%.17g", ex[extra_off[c.ci] + std::max(c.col, 0)]); break;
+          }
+          if (k) line += ' ';
+          line += buf;
+        }
+        line += '\n';
+        fputs(line.c_str(), f);
+      }
       fclose(f);
     }
   }
@@ -278,6 +394,7 @@ struct Shlmp {
     if (master()) printf("Loop time of %g on %d GPU%s for %lld steps with %zu atoms\n", rt, nranks, nranks > 1 ? "s" : "", (long long)nsteps, avec.nlocal());
     if (master()) printf("Pair  time (device) %g s in %lld launches | Neigh %g s in %lld builds | pair evals %lld | nodes evaluated %lld inside %lld\n",
            sp, (long long)pl, sn, (long long)nb, (long long)pe, (long long)ne, (long long)ni);
+    plan_extra({});
     pull_state();
   }
 };
@@ -322,6 +439,88 @@ void read_data(Shlmp &S, const std::string &fn) {
     }
   }
   if (natoms >= 0 && (long)S.avec.nlocal() != natoms) error_all(FLERR, "Did not assign all atoms correctly");
+}
+
+int find_compute(const Shlmp &S, const std::string &id) {
+  for (size_t k = 0; k < S.computes.size(); k++) if (S.computes[k].id == id) return (int)k;
+  return -1;
+}
+
+// compute ID all stress/atom NULL [ke] [pair] [virial] [branch center|centroid] | pe/atom [pair] | contact/atom
+void add_compute(Shlmp &S, const std::vector<std::string> &t) {
+  if (t.size() < 4) error_all(FLERR, "Illegal compute command");
+  if (t[2] != "all") error_all(FLERR, "Could not find compute group ID " + t[2]);
+  if (find_compute(S, t[1]) >= 0) error_all(FLERR, "Reuse of compute ID " + t[1]);
+  Compute c;
+  c.id = t[1];
+  const std::string &style = t[3];
+  if (style == "stress/atom") {
+    if (t.size() < 5) error_all(FLERR, "Illegal compute stress/atom command");
+    if (t[4] != "NULL") error_all(FLERR, "Could not find compute stress/atom temperature ID " + t[4]);
+    bool which = false, ke = false, pair = false;
+    for (size_t k = 5; k < t.size(); k++) {
+      if (t[k] == "ke") { ke = true; which = true; }
+      else if (t[k] == "pair" || t[k] == "virial") { pair = true; which = true; }
+      else if (t[k] == "branch" && k + 1 < t.size() && (t[k + 1] == "center" || t[k + 1] == "centroid")) c.mode = t[++k] == "centroid" ? 1 : 0;
+      else error_all(FLERR, "Illegal compute stress/atom command");
+    }
+    if (which) { c.ke = ke; c.pair = pair; }
+    c.style = Compute::STRESS;
+  } else if (style == "pe/atom") {
+    for (size_t k = 4; k < t.size(); k++) if (t[k] != "pair") error_all(FLERR, "Illegal compute pe/atom command");
+    c.style = Compute::PE;
+  } else if (style == "contact/atom") {
+    if (t.size() > 4) error_all(FLERR, "Illegal compute contact/atom command");
+    c.style = Compute::CONTACT;
+  } else {
+    error_all(FLERR, "Unknown compute style " + style);
+  }
+  S.computes.push_back(c);
+}
+
+// dump ID all custom N file [columns]; without columns the historic default list
+void add_dump(Shlmp &S, const std::vector<std::string> &t) {
+  if (t.size() < 6) error_all(FLERR, "Illegal dump command");
+  if (t[2] != "all") error_all(FLERR, "Could not find dump group ID " + t[2]);
+  Dump d;
+  d.every = std::stoi(t[4]); d.file = t[5];
+  std::vector<std::string> cols(t.begin() + 6, t.end());
+  if (cols.empty()) { std::istringstream is(kDefaultDumpCols); for (std::string w; is >> w;) cols.push_back(w); }
+  static const std::map<std::string, std::pair<DumpCol::Kind, int>> attrs = {
+      {"id", {DumpCol::ID, 0}}, {"type", {DumpCol::TYPE, 0}}, {"x", {DumpCol::X, 0}}, {"y", {DumpCol::X, 1}}, {"z", {DumpCol::X, 2}},
+      {"vx", {DumpCol::V, 0}}, {"vy", {DumpCol::V, 1}}, {"vz", {DumpCol::V, 2}}, {"qw", {DumpCol::Q, 0}}, {"qx", {DumpCol::Q, 1}},
+      {"qy", {DumpCol::Q, 2}}, {"qz", {DumpCol::Q, 3}}, {"fx", {DumpCol::F, 0}}, {"fy", {DumpCol::F, 1}}, {"fz", {DumpCol::F, 2}},
+      {"tqx", {DumpCol::TQ, 0}}, {"tqy", {DumpCol::TQ, 1}}, {"tqz", {DumpCol::TQ, 2}}, {"angmomx", {DumpCol::L, 0}},
+      {"angmomy", {DumpCol::L, 1}}, {"angmomz", {DumpCol::L, 2}}};
+  for (const std::string &a : cols) {
+    DumpCol col;
+    auto it = attrs.find(a);
+    if (it != attrs.end()) { col.kind = it->second.first; col.comp = it->second.second; }
+    else if (a.compare(0, 2, "c_") == 0 && a.size() > 2) {
+      std::string name = a.substr(2);
+      int idx = -1;
+      const size_t br = name.find('[');
+      if (br != std::string::npos) {
+        if (name.back() != ']' || br + 2 >= name.size()) error_all(FLERR, "Invalid attribute " + a + " in dump custom command");
+        const std::string num = name.substr(br + 1, name.size() - br - 2);
+        if (num.find_first_not_of("0123456789") != std::string::npos) error_all(FLERR, "Invalid attribute " + a + " in dump custom command");
+        idx = std::stoi(num);
+        name = name.substr(0, br);
+      }
+      const int ci = find_compute(S, name);
+      if (ci < 0) error_all(FLERR, "Could not find dump custom compute ID: " + name);
+      const int nc = S.computes[ci].ncols();
+      if (idx < 0 && nc > 0) error_all(FLERR, "Dump custom compute " + name + " does not calculate per-atom vector");
+      if (idx >= 0 && nc == 0) error_all(FLERR, "Dump custom compute " + name + " does not calculate per-atom array");
+      if (idx >= 0 && (idx < 1 || idx > nc)) error_all(FLERR, "Dump custom compute " + name + " vector is accessed out-of-range");
+      col.kind = DumpCol::COMP; col.ci = ci; col.col = idx - 1;
+    } else {
+      error_all(FLERR, "Invalid attribute " + a + " in dump custom command");
+    }
+    d.cols.push_back(col);
+    d.header += (d.header.empty() ? "" : " ") + a;
+  }
+  S.dumps.push_back(d);
 }
 
 void execute(Shlmp &S, const std::vector<std::string> &t) {
@@ -403,7 +602,8 @@ void execute(Shlmp &S, const std::vector<std::string> &t) {
   if (c == "neigh_modify") { for (size_t k = 1; k + 1 < t.size(); k += 2) { if (t[k] == "every") S.every = std::stoi(t[k + 1]); else if (t[k] == "check") S.check = t[k + 1] == "yes"; } return; }
   if (c == "timestep") { need(2); S.dt = std::stod(t[1]); if (!(S.dt > 0)) error_all(FLERR, "Illegal timestep command"); if (S.initialised && !S.dry) S.ck(sh_set_timestep(S.h, S.dt)); return; }
   if (c == "thermo") { need(2); S.thermo = std::stoi(t[1]); return; }
-  if (c == "dump") { need(6); Dump d; d.every = std::stoi(t[4]); d.file = t[5]; S.dumps.push_back(d); return; }
+  if (c == "compute") { add_compute(S, t); return; }
+  if (c == "dump") { add_dump(S, t); return; }
   if (c == "run") { need(2); S.run(std::stoll(t[1])); return; }
   if (c == "write_restart") {
     need(2); S.init();
