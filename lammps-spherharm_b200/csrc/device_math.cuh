@@ -20,6 +20,7 @@ struct DevShape {
   const double2 *ab;                      // folded (a,b) coefficients, m-major
   const double *px, *py, *pz;             // node points, shape frame
   const double *nx, *ny, *nz;             // oriented area elements n dS, shape frame
+  const double2 *pn;                      // the same per node in one 64 B record: (px,py) (pz,nx) (ny,nz) (0,0)
   int n_theta, n_phi;                     // node k = row*n_phi + col; phi_col = (col+1/2) 2pi/n_phi
   int tab_off;                            // offset (in records) of this shape in the concatenated table
   int nterms4;                            // nterms rounded up to a multiple of 4; tables hold nterms4+4 records

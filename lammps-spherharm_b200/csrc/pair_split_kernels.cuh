@@ -17,8 +17,9 @@
 //          shape-uniform whatever pair a record came from; persistent CTAs over contiguous chunks of the pools (the
 //          shape's folded table is staged in shared memory only when the shape changes), 2 or 4 points per lane sharing
 //          every coefficient load.  The work plan is computed ON THE DEVICE from the pool counters (no host round trip).
-//   C      pair_reduce_kernel  (small)  one thread per pair walks its two record runs in order (fixed order -> bitwise
-//          reproducible), accumulates the inside nodes, applies the contact law, writes the outputs.
+//   C      pair_reduce_kernel  (store bound)  a CTA takes 256 pairs, compacts those with nodes to sum in shared memory,
+//          and one thread per such pair walks its node indices in a fixed order (bitwise reproducible), accumulates the
+//          inside nodes, applies the contact law, writes the outputs; outputs that already hold zeros are not rewritten.
 // Pairs that do not fit (more than SURV_CAP staged survivors, or a full pool) go to a device list that the fused
 // warp kernel (pair_warp_kernel.cuh) processes afterwards: a full pool costs time, never correctness.
 // No floating-point atomics anywhere; pool offsets vary from run to run but never enter the arithmetic.
@@ -78,11 +79,14 @@ struct SplitScalars {
 
 struct SplitArgs {
   SurvRec *pool;                  // all shapes' pools in one buffer
-  unsigned char *pool_flag;       // inside flag per record (own array: a flag store must not dirty the 32 B record)
+  int *pool_kin;                  // per record: its node index if the node is inside, else -1 (own array: the reduction
+                                  // reads one contiguous int run per direction instead of the 32 B records)
   const long long *pool_base;     // [nshape] first record of the shape's pool
   const long long *pool_cap;      // [nshape]
   SplitScalars *sc;
   PdEntry *pd;                    // [2P] record run + inline inside nodes per (pair, direction)
+  unsigned char *out_zero;        // [P] 1: the pair's outputs (pres, both CSR slots) hold the zero record written by the
+                                  // reduction (cleared by the host whenever the list is rebuilt or another kernel wrote them)
   int *big_list;                  // [P]
   int *slow_list;                 // [P]
   int *inpool;                    // node indices proven inside by the cull beyond the inline capacity
@@ -564,7 +568,7 @@ __global__ void __launch_bounds__(WPB * 32, 32 / WPB) pair_cull_cached_kernel(Pa
         r.k = k; r.flag = fl;
         const long long idx = (dirc ? base1 : base0) + slot;
         S.pool[idx] = r;
-        S.pool_flag[idx] = 0;
+        S.pool_kin[idx] = -1;
       }
     }
     w0d0 += __popc(m0 & md0); w0d1 += __popc(m0 & ~md0);
@@ -715,8 +719,8 @@ __global__ void __launch_bounds__(WPB * 32) pair_cull_window_kernel(PairArgs A, 
       }
     } else {
       const long long base0 = S.pool_base[shp_j] + off0, base1 = S.pool_base[shp_i] + off1;
-      for (int r = lane; r < cnt0; r += 32) { S.pool[base0 + r] = s_rec[warp][0][r]; S.pool_flag[base0 + r] = s_rec[warp][0][r].flag == 2 ? 1 : 0; }
-      for (int r = lane; r < cnt1; r += 32) { S.pool[base1 + r] = s_rec[warp][1][r]; S.pool_flag[base1 + r] = s_rec[warp][1][r].flag == 2 ? 1 : 0; }
+      for (int r = lane; r < cnt0; r += 32) { const SurvRec q = s_rec[warp][0][r]; S.pool[base0 + r] = q; S.pool_kin[base0 + r] = q.flag == 2 ? q.k : -1; }
+      for (int r = lane; r < cnt1; r += 32) { const SurvRec q = s_rec[warp][1][r]; S.pool[base1 + r] = q; S.pool_kin[base1 + r] = q.flag == 2 ? q.k : -1; }
       if (lane == 0) store_pd(&S.pd[2 * p], base0, cnt0, nt0, nin0, s_in[warp][0]);
       if (lane == 1) store_pd(&S.pd[2 * p + 1], base1, cnt1, nt1, nin1, s_in[warp][1]);
     }
@@ -770,7 +774,7 @@ __global__ void __launch_bounds__(WPB * 32, MINB) pair_eval_kernel(const DevShap
     const long long r0 = ((long long)(blk - plan->blk_start[s]) * WPB + warp) * RPW;
     if (r0 >= n) continue;
     SurvRec *rec = S.pool + S.pool_base[s];
-    unsigned char *flg = S.pool_flag + S.pool_base[s];
+    int *kin = S.pool_kin + S.pool_base[s];
     const int L = sh.lmax;
     int nev = 0;
     if (PTS == 2) {
@@ -784,18 +788,18 @@ __global__ void __launch_bounds__(WPB * 32, MINB) pair_eval_kernel(const DevShap
         const double rhoB2 = fma(sB[2], sB[2], fma(sB[1], sB[1], sB[0] * sB[0]));
         double rhoA, rhoB, rA, rB;
         sh_radius_folded_x2(L, s_Ap, s_ab, sA, rhoA2, sB, rhoB2, rhoA, rhoB, rA, rB);
-        if (va && ra.flag == 0) { flg[ia] = rhoA < rA ? 1 : 0; nev++; }
-        if (vb && rb.flag == 0) { flg[ib] = rhoB < rB ? 1 : 0; nev++; }
+        if (va && ra.flag == 0) { kin[ia] = rhoA < rA ? ra.k : -1; nev++; }
+        if (vb && rb.flag == 0) { kin[ib] = rhoB < rB ? rb.k : -1; nev++; }
       } else if (va) {
         const SurvRec ra = rec[ia];
         const double rho2 = fma(ra.s2, ra.s2, fma(ra.s1, ra.s1, ra.s0 * ra.s0));
         double rho;
         const double r = sh_radius_folded(L, s_Ap, s_ab, ra.s0, ra.s1, ra.s2, rho2, rho);
-        if (ra.flag == 0) { flg[ia] = rho < r ? 1 : 0; nev++; }
+        if (ra.flag == 0) { kin[ia] = rho < r ? ra.k : -1; nev++; }
       }
     } else {
       double sv[PTS][3], rho2[PTS], rho[PTS], rr[PTS];
-      int fl[PTS];
+      int fl[PTS], kk[PTS];
       long long idx[PTS];
 #pragma unroll
       for (int q = 0; q < PTS; q++) {
@@ -804,12 +808,13 @@ __global__ void __launch_bounds__(WPB * 32, MINB) pair_eval_kernel(const DevShap
         const SurvRec r = rec[v ? idx[q] : r0];
         sv[q][0] = r.s0; sv[q][1] = r.s1; sv[q][2] = r.s2;
         fl[q] = v ? r.flag : 3;
+        kk[q] = r.k;
         rho2[q] = fma(r.s2, r.s2, fma(r.s1, r.s1, r.s0 * r.s0));
       }
       sh_radius_folded_n<PTS>(L, s_Ap, s_ab, sv, rho2, rho, rr);
 #pragma unroll
       for (int q = 0; q < PTS; q++)
-        if (fl[q] == 0) { flg[idx[q]] = rho[q] < rr[q] ? 1 : 0; nev++; }
+        if (fl[q] == 0) { kin[idx[q]] = rho[q] < rr[q] ? kk[q] : -1; nev++; }
     }
     nev_total += nev;
   }
@@ -818,14 +823,19 @@ __global__ void __launch_bounds__(WPB * 32, MINB) pair_eval_kernel(const DevShap
   if (lane == 0 && nev_total) { atomicAdd(&counters[2], nev_total); atomicAdd(&counters[5], nev_total); }
 }
 
-// ---- C: per-pair reduction + contact law (SURVEY A.5).  One THREAD per pair: the two record runs are short (a few
-// records, a few of them inside) and are summed sequentially in a fixed order: records of the run, then the inline
-// nodes.  Also the pair / transformed-node / ghost-pair counters of the cull kernels (one atomic per warp, not per pair).
+// ---- C: per-pair reduction + contact law (SURVEY A.5).  One THREAD per pair: the node lists are short (a few records, a
+// few of them inside) and each direction is summed sequentially in a fixed order: the records of the run, then the
+// index-pool run, then the inline nodes.  Fewer than half of the pairs have any node to sum: a CTA compacts those of its
+// 256 pairs in shared memory, so that its lanes are full while they sum.  The kernel is bound by its output stores (the
+// CSR slot of the reverse entry is a scattered 8 B store per component), and about 80 % of the pairs write the zero record
+// step after step: out_zero marks the pairs whose outputs already hold it, and their stores are skipped.  Deep-contact
+// pairs (cnt = -1) are done (and counted) by the fused kernel.
 struct NodeSums { double S0, S1, S2, Av, T0, T1, T2, G0, G1, G2; int n; };
 
-__device__ __forceinline__ void add_node(NodeSums &a, const double *__restrict__ nodes, int nq, int k, const double x0[3]) {
-  const double p0 = nodes[k], p1 = nodes[nq + k], p2 = nodes[2 * nq + k];
-  const double n0 = nodes[3 * nq + k], n1 = nodes[4 * nq + k], n2 = nodes[5 * nq + k];
+// one node of the packed table, (px,py) (pz,nx) (ny,nz); the same operations in the same order as the oracle
+__device__ __forceinline__ void add_node(NodeSums &a, double2 q0, double2 q1, double2 q2, const double x0[3]) {
+  const double p0 = q0.x, p1 = q0.y, p2 = q1.x;
+  const double n0 = q1.y, n1 = q2.x, n2 = q2.y;
   const double dp0 = p0 - x0[0], dp1 = p1 - x0[1], dp2 = p2 - x0[2];
   const double dn = fma(dp2, n2, fma(dp1, n1, dp0 * n0));
   a.S0 += n0; a.S1 += n1; a.S2 += n2;
@@ -837,150 +847,185 @@ __device__ __forceinline__ void add_node(NodeSums &a, const double *__restrict__
   a.n++;
 }
 
-template <int MINB>
-__global__ void __launch_bounds__(128, MINB) pair_reduce_kernel(PairArgs A, SplitArgs S) {
-  const int p = blockIdx.x * blockDim.x + threadIdx.x;
-  int c_pairs = 0, c_trans = 0, c_inside = 0, c_ghost = 0;
-  if (p < A.npairs) {
+// the 14-double pair record (coalesced across pairs) and the force / torque of the pair's two CSR slots
+__device__ __forceinline__ void store_pair_outputs(const PairArgs &A, int p, const double out[14]) {
+#pragma unroll
+  for (int r = 0; r < 14; r++) A.pres[(size_t)r * A.pres_stride + p] = out[r];
+  const int eij = A.pair_eij[p], eji = A.pair_eji[p];
+#pragma unroll
+  for (int r = 0; r < 3; r++) {
+    A.slot[(size_t)r * A.slot_stride + eij] = out[2 + r];
+    A.slot[(size_t)(3 + r) * A.slot_stride + eij] = out[5 + r];
+    if (eji >= 0) {
+      A.slot[(size_t)r * A.slot_stride + eji] = -out[2 + r];
+      A.slot[(size_t)(3 + r) * A.slot_stride + eji] = out[8 + r];
+    }
+  }
+}
+
+// writes the pair's outputs unless they are zero and already hold zeros
+__device__ __forceinline__ void store_pair_outputs_once(const PairArgs &A, const SplitArgs &S, int p, bool zero, const double out[14]) {
+  const bool held = S.out_zero[p] != 0;
+  if (zero && held) return;
+  store_pair_outputs(A, p, out);
+  if (zero != held) S.out_zero[p] = zero ? 1 : 0;
+}
+
+// one pair with nodes to sum.  Per direction the node indices come from three sources in order (run records through
+// pool_kin, index pool, inline); RB of them are fetched, then their nodes loaded, then summed in order, so that a pair's
+// node loads are in flight together.  Returns the number of inside nodes.
+__device__ __forceinline__ int reduce_contact_pair(const PairArgs &A, const SplitArgs &S, int p) {
+  constexpr int RB = 2;
+  {
     const int4 *ep = reinterpret_cast<const int4 *>(S.pd + 2 * (size_t)p);
     const int4 e0a = __ldg(ep), e0b = __ldg(ep + 1), e1a = __ldg(ep + 2), e1b = __ldg(ep + 3);
-    const int cnt0 = e0a.z, cnt1 = e1a.z;
-    if (cnt0 >= 0) {   // else: deep contact, done (and counted) by the fused kernel
-      const int i = A.pair_i[p], j = A.pair_j[p];
-      c_pairs = 1; c_trans = (e0a.w & 0xffff) + (e1a.w & 0xffff); c_ghost = j >= A.nlocal;
-      const int nin0 = e0b.y & 0xffff, nin1 = e1b.y & 0xffff;
-      const int xc0 = (e0a.w >> 16) & 0xffff, xc1 = (e1a.w >> 16) & 0xffff;     // proven-inside nodes in the index pool
-      double out[14];
+    const int i = A.pair_i[p], j = A.pair_j[p];
+    const int st = A.stride;
+    double d[3];
+    pair_separation(A, p, i, j, d);
+    const int shp_i = A.shape[i], shp_j = A.shape[j];
+    double out[14];
 #pragma unroll
-      for (int r = 0; r < 14; r++) out[r] = 0.0;
-      // inside flags of both runs first (independent loads), as bit masks
-      const long long off0 = (long long)(((unsigned long long)(unsigned)e0a.y << 32) | (unsigned)e0a.x);
-      const long long off1 = (long long)(((unsigned long long)(unsigned)e1a.y << 32) | (unsigned)e1a.x);
-      unsigned long long msk0 = 0, msk1 = 0;
-      bool any = nin0 > 0 || nin1 > 0 || xc0 > 0 || xc1 > 0;
-      {
-        const int m0 = min(cnt0, 64), m1 = min(cnt1, 64);
-        for (int r = 0; r < m0; r += 8) {
+    for (int r = 0; r < 14; r++) out[r] = 0.0;
+    double Ss[2][3], Ts[2][3], Gs[2][3], Asum[2];
+    int ninside_pair = 0;
 #pragma unroll
-          for (int q = 0; q < 8; q++) if (r + q < m0 && S.pool_flag[off0 + r + q]) msk0 |= 1ull << (r + q);
-        }
-        for (int r = 0; r < m1; r += 8) {
+    for (int dir = 0; dir < 2; dir++) {
+      const int a = dir ? j : i;
+      const DevShape &sa = A.shapes[dir ? shp_j : shp_i];
+      const double sgn = dir ? -1.0 : 1.0;
+      const int4 ea = dir ? e1a : e0a, eb = dir ? e1b : e0b;
+      const long long off = (long long)(((unsigned long long)(unsigned)ea.y << 32) | (unsigned)ea.x);
+      const int cnt = ea.z, xc = (ea.w >> 16) & 0xffff, nin = eb.y & 0xffff;   // run records, index-pool and inline nodes
+      const int nrx = cnt + xc, ntot = nrx + nin;
+      const int *__restrict__ kin = S.pool_kin + off;
+      const int *__restrict__ xin = S.inpool + (unsigned)eb.x;
+      const double2 *__restrict__ pn = sa.pn;
+      NodeSums acc;
+      acc.S0 = acc.S1 = acc.S2 = acc.Av = acc.T0 = acc.T1 = acc.T2 = acc.G0 = acc.G1 = acc.G2 = 0.0; acc.n = 0;
+      double Ra[9];
 #pragma unroll
-          for (int q = 0; q < 8; q++) if (r + q < m1 && S.pool_flag[off1 + r + q]) msk1 |= 1ull << (r + q);
-        }
-        any = any || msk0 || msk1 || cnt0 > 64 || cnt1 > 64;
-      }
-      if (any) {
-        const int st = A.stride;
-        double d[3];
-        pair_separation(A, p, i, j, d);
-        const int shp_i = A.shape[i], shp_j = A.shape[j];
-        double Ss[2][3], Ts[2][3], Gs[2][3], Asum[2];
-        int ninside_pair = 0;
-#pragma unroll
-        for (int dir = 0; dir < 2; dir++) {
-          const int a = dir ? j : i;
-          const DevShape &sa = A.shapes[dir ? shp_j : shp_i];
-          const double sgn = dir ? -1.0 : 1.0;
-          const long long off = dir ? off1 : off0;
-          const int cnt = dir ? cnt1 : cnt0, nin = dir ? nin1 : nin0, xc = dir ? xc1 : xc0;
-          unsigned long long msk = dir ? msk1 : msk0;
-          const int4 eb = dir ? e1b : e0b;
-          NodeSums acc;
-          acc.S0 = acc.S1 = acc.S2 = acc.Av = acc.T0 = acc.T1 = acc.T2 = acc.G0 = acc.G1 = acc.G2 = 0.0; acc.n = 0;
-          double Ra[9];
-#pragma unroll
-          for (int e = 0; e < 9; e++) Ra[e] = A.Rs[e * st + a];
-          if (msk || nin > 0 || cnt > 64 || xc > 0) {
-            double x0[3];
-#pragma unroll
-            for (int r = 0; r < 3; r++) {
-              double hx = Ra[0 + r] * (sgn * d[0]);
-              hx = fma(Ra[3 + r], sgn * d[1], hx);
-              hx = fma(Ra[6 + r], sgn * d[2], hx);
-              x0[r] = -0.5 * hx;
-            }
-            const double *__restrict__ nodes = sa.px;
-            const int nq = sa.nq;
-            while (msk) {   // records of the run, in order
-              const int r = __ffsll((long long)msk) - 1;
-              msk &= msk - 1;
-              add_node(acc, nodes, nq, S.pool[off + r].k, x0);
-            }
-            for (int r = 64; r < cnt; r++)
-              if (S.pool_flag[off + r]) add_node(acc, nodes, nq, S.pool[off + r].k, x0);
-            // nodes proven inside by the cull: the index-pool run, then the inline ones, in order
-            {
-              const unsigned xo = (unsigned)eb.x;
-              for (int r = 0; r < xc; r++) add_node(acc, nodes, nq, S.inpool[xo + r], x0);
-            }
-            for (int q = 0; q < nin; q++) {
-              const int h = q + 3;                       // halfword index inside the second 16 B of the entry (off2, nin, in[])
-              const unsigned w = (h >> 1) == 0 ? (unsigned)eb.x : (h >> 1) == 1 ? (unsigned)eb.y : (h >> 1) == 2 ? (unsigned)eb.z : (unsigned)eb.w;
-              add_node(acc, nodes, nq, (int)((w >> (16 * (h & 1))) & 0xffffu), x0);
-            }
-          }
-#pragma unroll
-          for (int r = 0; r < 3; r++) {
-            Ss[dir][r] = Ra[3 * r] * acc.S0 + Ra[3 * r + 1] * acc.S1 + Ra[3 * r + 2] * acc.S2;
-            Ts[dir][r] = Ra[3 * r] * acc.T0 + Ra[3 * r + 1] * acc.T1 + Ra[3 * r + 2] * acc.T2;
-            Gs[dir][r] = 0.25 * (Ra[3 * r] * acc.G0 + Ra[3 * r + 1] * acc.G1 + Ra[3 * r + 2] * acc.G2);
-          }
-          Asum[dir] = acc.Av;
-          ninside_pair += acc.n;
-        }
-        c_inside = ninside_pair;
-        const double V = Asum[0] / 3.0 + Asum[1] / 3.0;
-        if (ninside_pair > 0 && V > 0) {
-          const double kk = A.pk[shp_i * SH_MAX_SHAPES + shp_j], mm = A.pm[shp_i * SH_MAX_SHAPES + shp_j];
-          double E, pr;
-          if (mm == 1.0) { E = kk * V; pr = kk; }
-          else { const double pw = pow(V, mm - 1.0); E = kk * pw * V; pr = mm * kk * pw; }
-          out[0] = V; out[1] = E;
-          double li[3], lj[3];
-#pragma unroll
-          for (int r = 0; r < 3; r++) {
-            li[r] = A.c[r * st + i] - A.x[r * st + i];
-            lj[r] = A.c[r * st + j] - A.x[r * st + j];
-          }
-          const double *Sij = Ss[0], *Sji = Ss[1], *Tij = Ts[0], *Tji = Ts[1];
-          const double Ti[3] = {Tij[0] + (li[1] * Sij[2] - li[2] * Sij[1]), Tij[1] + (li[2] * Sij[0] - li[0] * Sij[2]),
-                                Tij[2] + (li[0] * Sij[1] - li[1] * Sij[0])};
-          const double Tj[3] = {Tji[0] + (lj[1] * Sji[2] - lj[2] * Sji[1]), Tji[1] + (lj[2] * Sji[0] - lj[0] * Sji[2]),
-                                Tji[2] + (lj[0] * Sji[1] - lj[1] * Sji[0])};
-#pragma unroll
-          for (int r = 0; r < 3; r++) {
-            out[2 + r] = -pr * (0.5 * (Sij[r] - Sji[r]));
-            out[5 + r] = -pr * Ti[r];
-            out[8 + r] = -pr * Tj[r];
-            out[11 + r] = (A.c[r * st + i] - 0.5 * d[r]) + (Gs[0][r] + Gs[1][r]) / V;
-          }
-          if (A.dissip) contact_dissipation(A, i, j, shp_i, shp_j, d, lj, out);
-        }
-      }
-#pragma unroll
-      for (int r = 0; r < 14; r++) A.pres[(size_t)r * A.pres_stride + p] = out[r];   // coalesced across pairs
-      const int eij = A.pair_eij[p], eji = A.pair_eji[p];
+      for (int e = 0; e < 9; e++) Ra[e] = A.Rs[e * st + a];
+      double x0[3];
 #pragma unroll
       for (int r = 0; r < 3; r++) {
-        A.slot[(size_t)r * A.slot_stride + eij] = out[2 + r];
-        A.slot[(size_t)(3 + r) * A.slot_stride + eij] = out[5 + r];
-        if (eji >= 0) {
-          A.slot[(size_t)r * A.slot_stride + eji] = -out[2 + r];
-          A.slot[(size_t)(3 + r) * A.slot_stride + eji] = out[8 + r];
-        }
+        double hx = Ra[0 + r] * (sgn * d[0]);
+        hx = fma(Ra[3 + r], sgn * d[1], hx);
+        hx = fma(Ra[6 + r], sgn * d[2], hx);
+        x0[r] = -0.5 * hx;
       }
+      for (int b = 0; b < ntot; b += RB) {
+        int k[RB];
+#pragma unroll
+        for (int u = 0; u < RB; u++) {
+          const int g = b + u;
+          if (g < cnt) k[u] = kin[g];                  // -1: the record's node is outside
+          else if (g < nrx) k[u] = xin[g - cnt];
+          else if (g < ntot) {
+            const int h = g - nrx + 3;                 // halfword index inside the second 16 B of the entry (off2, nin, in[])
+            const unsigned w = (h >> 1) == 1 ? (unsigned)eb.y : (h >> 1) == 2 ? (unsigned)eb.z : (unsigned)eb.w;
+            k[u] = (int)((w >> (16 * (h & 1))) & 0xffffu);
+          } else k[u] = -1;
+        }
+        double2 q[RB][3];
+#pragma unroll
+        for (int u = 0; u < RB; u++) {
+          if (k[u] >= 0) { q[u][0] = pn[4 * k[u]]; q[u][1] = pn[4 * k[u] + 1]; q[u][2] = pn[4 * k[u] + 2]; }
+          else q[u][0] = q[u][1] = q[u][2] = make_double2(0.0, 0.0);
+        }
+#pragma unroll
+        for (int u = 0; u < RB; u++)
+          if (k[u] >= 0) add_node(acc, q[u][0], q[u][1], q[u][2], x0);
+      }
+#pragma unroll
+      for (int r = 0; r < 3; r++) {
+        Ss[dir][r] = Ra[3 * r] * acc.S0 + Ra[3 * r + 1] * acc.S1 + Ra[3 * r + 2] * acc.S2;
+        Ts[dir][r] = Ra[3 * r] * acc.T0 + Ra[3 * r + 1] * acc.T1 + Ra[3 * r + 2] * acc.T2;
+        Gs[dir][r] = 0.25 * (Ra[3 * r] * acc.G0 + Ra[3 * r + 1] * acc.G1 + Ra[3 * r + 2] * acc.G2);
+      }
+      Asum[dir] = acc.Av;
+      ninside_pair += acc.n;
     }
+    const double V = Asum[0] / 3.0 + Asum[1] / 3.0;
+    const bool contact = ninside_pair > 0 && V > 0;
+    if (contact) {
+      const double kk = A.pk[shp_i * SH_MAX_SHAPES + shp_j], mm = A.pm[shp_i * SH_MAX_SHAPES + shp_j];
+      double E, pr;
+      if (mm == 1.0) { E = kk * V; pr = kk; }
+      else { const double pw = pow(V, mm - 1.0); E = kk * pw * V; pr = mm * kk * pw; }
+      out[0] = V; out[1] = E;
+      double li[3], lj[3];
+#pragma unroll
+      for (int r = 0; r < 3; r++) {
+        li[r] = A.c[r * st + i] - A.x[r * st + i];
+        lj[r] = A.c[r * st + j] - A.x[r * st + j];
+      }
+      const double *Sij = Ss[0], *Sji = Ss[1], *Tij = Ts[0], *Tji = Ts[1];
+      const double Ti[3] = {Tij[0] + (li[1] * Sij[2] - li[2] * Sij[1]), Tij[1] + (li[2] * Sij[0] - li[0] * Sij[2]),
+                            Tij[2] + (li[0] * Sij[1] - li[1] * Sij[0])};
+      const double Tj[3] = {Tji[0] + (lj[1] * Sji[2] - lj[2] * Sji[1]), Tji[1] + (lj[2] * Sji[0] - lj[0] * Sji[2]),
+                            Tji[2] + (lj[0] * Sji[1] - lj[1] * Sji[0])};
+#pragma unroll
+      for (int r = 0; r < 3; r++) {
+        out[2 + r] = -pr * (0.5 * (Sij[r] - Sji[r]));
+        out[5 + r] = -pr * Ti[r];
+        out[8 + r] = -pr * Tj[r];
+        out[11 + r] = (A.c[r * st + i] - 0.5 * d[r]) + (Gs[0][r] + Gs[1][r]) / V;
+      }
+      if (A.dissip) contact_dissipation(A, i, j, shp_i, shp_j, d, lj, out);
+    }
+    store_pair_outputs_once(A, S, p, !contact, out);
+    return ninside_pair;
+  }
+}
+
+__global__ void __launch_bounds__(128, 4) pair_reduce_kernel(PairArgs A, SplitArgs S) {
+  constexpr int PPT = 2;   // pairs per thread in the CTA's range
+  __shared__ int s_list[PPT * 128];
+  __shared__ int s_n;
+  if (threadIdx.x == 0) s_n = 0;
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  int c_pairs = 0, c_trans = 0, c_ghost = 0;
+#pragma unroll
+  for (int q = 0; q < PPT; q++) {
+    const int p = (blockIdx.x * PPT + q) * 128 + threadIdx.x;
+    bool hit = false;
+    if (p < A.npairs) {
+      const int4 *ep = reinterpret_cast<const int4 *>(S.pd + 2 * (size_t)p);
+      const int4 e0a = __ldg(ep), e0b = __ldg(ep + 1), e1a = __ldg(ep + 2), e1b = __ldg(ep + 3);
+      if (e0a.z >= 0) {
+        c_pairs++; c_trans += (e0a.w & 0xffff) + (e1a.w & 0xffff); c_ghost += A.pair_j[p] >= A.nlocal;
+        // records, index-pool or inline inside nodes in either direction
+        hit = e0a.z + e1a.z + ((e0a.w >> 16) & 0xffff) + ((e1a.w >> 16) & 0xffff) + (e0b.y & 0xffff) + (e1b.y & 0xffff) > 0;
+        if (!hit) {
+          double out[14];
+#pragma unroll
+          for (int r = 0; r < 14; r++) out[r] = 0.0;
+          store_pair_outputs_once(A, S, p, true, out);
+        }
+      } else if (S.out_zero[p]) S.out_zero[p] = 0;   // the fused kernel writes this pair's outputs
+    }
+    const unsigned m = __ballot_sync(0xffffffffu, hit);
+    int base = 0;
+    if (lane == 0 && m) base = atomicAdd(&s_n, __popc(m));
+    base = __shfl_sync(0xffffffffu, base, 0);
+    if (hit) s_list[base + __popc(m & ((1u << lane) - 1u))] = p;
   }
   // counters: one atomic per warp and counter
   c_pairs = __reduce_add_sync(0xffffffffu, c_pairs); c_trans = __reduce_add_sync(0xffffffffu, c_trans);
-  c_inside = __reduce_add_sync(0xffffffffu, c_inside); c_ghost = __reduce_add_sync(0xffffffffu, c_ghost);
-  if ((threadIdx.x & 31) == 0) {
+  c_ghost = __reduce_add_sync(0xffffffffu, c_ghost);
+  if (lane == 0) {
     if (c_pairs) atomicAdd(&A.counters[0], (unsigned long long)c_pairs);
     if (c_trans) atomicAdd(&A.counters[1], (unsigned long long)c_trans);
-    if (c_inside) atomicAdd(&A.counters[3], (unsigned long long)c_inside);
     if (c_ghost) atomicAdd(&A.counters[4], (unsigned long long)c_ghost);
   }
+  __syncthreads();
+  const int n = s_n;
+  int c_inside = 0;
+  for (int t = threadIdx.x; t < n; t += 128) c_inside += reduce_contact_pair(A, S, s_list[t]);
+  c_inside = __reduce_add_sync(0xffffffffu, c_inside);
+  if (lane == 0 && c_inside) atomicAdd(&A.counters[3], (unsigned long long)c_inside);
 }
 
 }  // namespace shgpu

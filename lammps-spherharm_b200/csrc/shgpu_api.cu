@@ -30,7 +30,7 @@ namespace {
 
 struct ShapeDev {
   DevBuf<double> Ap, node;   // node: 6 x nq
-  DevBuf<double2> ab;
+  DevBuf<double2> ab, pn;    // pn: packed node records for the pair reduction (DevShape::pn)
   DevBuf<float> row_x, cubew[SH_CACHE_LEVELS];
   DevBuf<float2> cube;       // {ub2, lb2} per direction cell
   DevBuf<float4> pf4;        // FP32 node points
@@ -93,7 +93,9 @@ struct sh_ctx {
   DevBuf<double> bbox, slot, pres, stage;
   // split pair pipeline (pair_split_kernels.cuh)
   DevBuf<SurvRec> pool;
-  DevBuf<unsigned char> pool_flag;
+  DevBuf<int> pool_kin;
+  DevBuf<unsigned char> out_zero;                 // SplitArgs::out_zero; valid only while out_zero_valid
+  bool out_zero_valid = false;                     // cleared by a list build and by every pair phase outside run_split_pipeline
   DevBuf<long long> pool_base, pool_cap;
   DevBuf<PdEntry> pd;
   DevBuf<PairHot> cache_hot[2];       // double-buffered: a neighbor rebuild remaps the live cache into the other buffer
@@ -116,7 +118,6 @@ struct sh_ctx {
   int64_t cache_age = 0;                       // pair phases since the last cache build
   bool cache_exhausted = false;                // the last invalidation came from the displacement margin
   int cube_n = 0;                              // direction cells per cube-face edge (0 = default)
-  int reduce_occ = 0;
   int eval_pts = 0, eval_occ = 0, eval_mode = 0;   // pair_eval_kernel: points per lane, min CTAs/SM, 1 = one block per CTA
   long long last_records = 0;                  // records of the previous pair phase (advisory)
   // candidate cache
@@ -213,6 +214,17 @@ int upload_shapes(sh_ctx *h) {
         CU(cudaMemcpy(d.node.p + (size_t)e * t.nq, t.node_p[e].data(), t.nq * sizeof(double), cudaMemcpyHostToDevice));
         CU(cudaMemcpy(d.node.p + (size_t)(3 + e) * t.nq, t.node_n[e].data(), t.nq * sizeof(double), cudaMemcpyHostToDevice));
       }
+      {
+        std::vector<double2> pn((size_t)4 * t.nq);
+        for (int k = 0; k < t.nq; k++) {
+          pn[4 * (size_t)k] = make_double2(t.node_p[0][k], t.node_p[1][k]);
+          pn[4 * (size_t)k + 1] = make_double2(t.node_p[2][k], t.node_n[0][k]);
+          pn[4 * (size_t)k + 2] = make_double2(t.node_n[1][k], t.node_n[2][k]);
+          pn[4 * (size_t)k + 3] = make_double2(0.0, 0.0);
+        }
+        d.pn.ensure(pn.size());
+        CU(cudaMemcpy(d.pn.p, pn.data(), pn.size() * sizeof(double2), cudaMemcpyHostToDevice));
+      }
       DevShape &v = h->shape_host_view[s];
       v.lmax = t.lmax; v.nterms = t.nterms; v.nq = t.nq; v.nchunks = (t.nq + 31) / 32;
       v.rmax = t.rmax; v.rmin = t.rmin; v.rmax2 = t.rmax * t.rmax; v.rmin2 = t.rmin * t.rmin;
@@ -222,6 +234,7 @@ int upload_shapes(sh_ctx *h) {
       v.Ap = d.Ap.p; v.ab = d.ab.p;
       v.px = d.node.p; v.py = d.node.p + t.nq; v.pz = d.node.p + 2 * (size_t)t.nq;
       v.nx = d.node.p + 3 * (size_t)t.nq; v.ny = d.node.p + 4 * (size_t)t.nq; v.nz = d.node.p + 5 * (size_t)t.nq;
+      v.pn = d.pn.p;
       v.n_theta = t.n_theta; v.n_phi = t.n_phi; v.nterms4 = (t.nterms + 3) / 4 * 4; v.row_x = d.row_x.p; v.cube_ul = d.cube.p; v.cube_n = t.cube_n; v.pad2_ = 0; v.pf4 = d.pf4.p;
       for (int lv = 0; lv < SH_CACHE_LEVELS; lv++) { v.cube_w2[lv] = d.cubew[lv].p; v.cache_delta[lv] = t.cache_delta[lv]; }
     }
@@ -375,6 +388,7 @@ int build_neighbors(sh_ctx *h) {
   CU(cudaGetLastError());
   h->npairs = npairs; h->nentries = nentries;
   h->list_valid = true; h->steps_since_build = 0; h->neighbor_builds++;
+  h->out_zero_valid = false;   // new pairs and CSR entries
   // the pair list changed: a live cache over the same atoms is remapped, anything else is rebuilt
   h->cache_state = keep_cache ? CACHE_REMAP : CACHE_INVALID;
   if (!keep_cache) h->carry = false;
@@ -498,6 +512,7 @@ int run_split_pipeline(sh_ctx *h, PairArgs &P) {
   if ((rc = absorb_split_feedback(h))) return rc;
   try {
     h->pd.ensure((size_t)2 * np + 2); h->big_list.ensure(np + 1); h->slow_list.ensure(np + 1);
+    if (h->out_zero.cap < (size_t)np + 1) { h->out_zero.ensure(np + 1); h->out_zero_valid = false; }
     h->pool_base.ensure(SH_MAX_SHAPES); h->pool_cap.ensure(SH_MAX_SHAPES); h->split_sc.ensure(1); h->eval_plan.ensure(1); h->split_flags.ensure(4);
   } catch (std::string &e) { return fail(h, e); }
   if (!h->h_pool_count) {
@@ -616,13 +631,13 @@ int run_split_pipeline(sh_ctx *h, PairArgs &P) {
   for (int s2 = 0; s2 < ns; s2++) { base[s2] = tot; tot += h->h_pool_cap[s2]; }
   if (h->h_in_cap < (long long)np * 2 + 4096) h->h_in_cap = (long long)np * 2 + 4096;
   if (h->h_in_cap > 0xfffffff0LL) h->h_in_cap = 0xfffffff0LL;      // 32-bit offsets in the run descriptors
-  try { h->pool.ensure((size_t)tot + 64); h->pool_flag.ensure((size_t)tot + 64); h->inpool.ensure((size_t)h->h_in_cap + 64); } catch (std::string &e) { return fail(h, e); }
+  try { h->pool.ensure((size_t)tot + 64); h->pool_kin.ensure((size_t)tot + 64); h->inpool.ensure((size_t)h->h_in_cap + 64); } catch (std::string &e) { return fail(h, e); }
   CU(cudaMemcpyAsync(h->pool_base.p, base.data(), ns * sizeof(long long), cudaMemcpyHostToDevice, h->stream));
   CU(cudaMemcpyAsync(h->pool_cap.p, h->h_pool_cap.data(), ns * sizeof(long long), cudaMemcpyHostToDevice, h->stream));
   CU(cudaMemsetAsync(h->split_sc.p, 0, sizeof(SplitScalars), h->stream));
   SplitArgs S;
-  S.pool = h->pool.p; S.pool_flag = h->pool_flag.p; S.pool_base = h->pool_base.p; S.pool_cap = h->pool_cap.p; S.sc = h->split_sc.p;
-  S.pd = h->pd.p; S.big_list = h->big_list.p; S.slow_list = h->slow_list.p; S.inpool = h->inpool.p; S.in_cap = h->h_in_cap;
+  S.pool = h->pool.p; S.pool_kin = h->pool_kin.p; S.pool_base = h->pool_base.p; S.pool_cap = h->pool_cap.p; S.sc = h->split_sc.p;
+  S.pd = h->pd.p; S.out_zero = h->out_zero.p; S.big_list = h->big_list.p; S.slow_list = h->slow_list.p; S.inpool = h->inpool.p; S.in_cap = h->h_in_cap;
   // ---- A
   if (tick(0)) return -2;
   if (C.enabled) {
@@ -660,9 +675,11 @@ int run_split_pipeline(sh_ctx *h, PairArgs &P) {
   h->eval_launches++;
   // ---- C
   if (tick(2)) return -2;
-  if (h->reduce_occ == 4) pair_reduce_kernel<4><<<cdiv(np, 128), 128, 0, h->stream>>>(P, S);
-  else if (h->reduce_occ == 8) pair_reduce_kernel<8><<<cdiv(np, 128), 128, 0, h->stream>>>(P, S);
-  else pair_reduce_kernel<6><<<cdiv(np, 128), 128, 0, h->stream>>>(P, S);
+  if (!h->out_zero_valid) {   // nothing is known about the outputs' contents
+    CU(cudaMemsetAsync(h->out_zero.p, 0, (size_t)np, h->stream));
+    h->out_zero_valid = true;
+  }
+  pair_reduce_kernel<<<cdiv(np, 256), 128, 0, h->stream>>>(P, S);
   tock();
   h->kernel_launches++;
   // ---- deep contacts / pairs that found the pool full: fused kernel over the device-side list
@@ -708,12 +725,14 @@ int compute_forces_device(sh_ctx *h) {
     CU(cudaEventRecord(h->ev[h->ev_used], h->stream));
     int rc;
     if (h->tune_variant & 1) {           // CTA-per-pair kernel (full-table scan)
+      h->out_zero_valid = false;
       if (nt == 256) rc = launch_pair<256>(h, P, h->tune_ctas_per_sm, pair_smem_bytes(maxT, maxq, 8));
       else if (nt == 64) rc = launch_pair<64>(h, P, h->tune_ctas_per_sm, pair_smem_bytes(maxT, maxq, 2));
       else rc = launch_pair<128>(h, P, h->tune_ctas_per_sm, pair_smem_bytes(maxT, maxq, 4));
     } else if ((h->tune_variant & 4) || (!(h->tune_variant & 16) && h->npairs < 16384)) {
       // fused warp-per-pair kernel: explicit (bit 4), or small systems where the split pipeline's extra
       // launches and its host sync cost more than they save (bit 16 forces the split pipeline)
+      h->out_zero_valid = false;
       rc = launch_fused(h, P);
     } else {                             // split pipeline (default): cull / evaluate / reduce
       rc = run_split_pipeline(h, P);
@@ -856,7 +875,7 @@ int sh_destroy(sh_ctx *h) {
   if (!h) return 0;
   cudaSetDevice(h->device);
   cudaStreamSynchronize(h->stream);
-  for (auto &d : h->shape_dev) { d.Ap.release(); d.ab.release(); d.node.release(); d.row_x.release(); d.cube.release(); d.pf4.release(); for (auto &w : d.cubew) w.release(); }
+  for (auto &d : h->shape_dev) { d.Ap.release(); d.ab.release(); d.node.release(); d.row_x.release(); d.cube.release(); d.pf4.release(); d.pn.release(); for (auto &w : d.cubew) w.release(); }
   h->d_shapes.release(); h->d_pk.release(); h->d_pm.release(); h->d_pgn.release(); h->d_pgt.release(); h->d_pmu.release(); h->stress_part.release();
   DevBuf<double> *db[] = {&h->x, &h->v, &h->q, &h->L, &h->f, &h->tq, &h->c, &h->Rs, &h->c0, &h->wallf, &h->ewall, &h->ke, &h->bbox, &h->slot, &h->pres};
   for (auto *b : db) b->release();
@@ -867,8 +886,8 @@ int sh_destroy(sh_ctx *h) {
   h->as_vir.release(); h->as_kin.release(); h->as_en.release(); h->as_send.release(); h->as_recv.release(); h->as_cnt.release(); h->as_epair.release();
   for (auto &e : h->ev) cudaEventDestroy(e);
   for (auto &e : h->ev2) cudaEventDestroy(e);
-  h->pool.release(); h->pool_flag.release(); h->pool_base.release(); h->pool_cap.release(); h->split_sc.release(); h->eval_plan.release(); h->slow_list.release();
-  h->pd.release(); h->big_list.release(); h->split_flags.release(); h->inpool.release();
+  h->pool.release(); h->pool_kin.release(); h->pool_base.release(); h->pool_cap.release(); h->split_sc.release(); h->eval_plan.release(); h->slow_list.release();
+  h->pd.release(); h->out_zero.release(); h->big_list.release(); h->split_flags.release(); h->inpool.release();
   for (int k = 0; k < 2; k++) { h->cache_hot[k].release(); h->cache_pool[k].release(); }
   h->old_c.release(); h->old_cc0.release(); h->old_cq0.release(); h->old_tag.release(); h->ghost_hash.release(); h->amap.release();
   h->old_half_off.release(); h->old_pair_j.release(); h->fresh_list.release(); h->cache_count.release(); h->cc0.release(); h->cq0.release(); h->drift.release();
@@ -1710,7 +1729,6 @@ int sh_set_tuning(sh_ctx *h, const char *key, double value) try {
   const int v = (int)value;
   if (k == "cull_wpb") { if (v != 0 && v != 1 && v != 2 && v != 4 && v != 8) return fail(h, "cull_wpb must be 0, 1, 2, 4 or 8"); h->tune_cull_wpb = v; }
   else if (k == "cull_lpp") { if (v != 0 && v != 16 && v != 32) return fail(h, "cull_lpp must be 0, 16 or 32"); h->tune_cull_lpp = v; }
-  else if (k == "reduce_occ") { if (v != 0 && v != 4 && v != 6 && v != 8) return fail(h, "reduce_occ must be 0, 4, 6 or 8"); h->reduce_occ = v; }
   else if (k == "eval_pts") { if (v != 0 && v != 2 && v != 4) return fail(h, "eval_pts must be 0, 2 or 4"); h->eval_pts = v; }
   else if (k == "eval_occ") { if (v != 0 && v != 3 && v != 4) return fail(h, "eval_occ must be 0, 3 or 4"); h->eval_occ = v; }
   else if (k == "eval_mode") { if (v < 0 || v > 2) return fail(h, "eval_mode must be 0 (default), 1 (one block per CTA) or 2 (persistent chunks)"); h->eval_mode = v; }
