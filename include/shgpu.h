@@ -55,6 +55,14 @@ int sh_pair_dissipation(sh_ctx *h, int shape_i, int shape_j, double gamma_n, dou
 /* fix wall for SH particles (Fix::post_force): plane through point, normal into the domain -- */
 int sh_add_wall(sh_ctx *h, const double point[3], const double normal[3], double k,
                 double exponent);
+/* curved container walls (fix wall/spherharm zcylinder | sphere; LAMMPS fix wall/gran ... zcylinder): static and elastic,
+ * with the plane wall's contact law E = k V^exponent on the volume V of the particle outside the wall.  The particles are
+ * INSIDE.  Cylinder: infinite, axis the line through `point` along `axis` (any direction, any nonzero length).  Sphere:
+ * centre `center`.  Up to 8 curved walls, applied after the plane walls in insertion order; refused: a zero axis,
+ * radius <= 0, k < 0, exponent < 1, a 9th curved wall.  Only owned atoms get wall force; walls add no virial. */
+int sh_add_cylinder_wall(sh_ctx *h, const double point[3], const double axis[3], double radius, double k,
+                         double exponent);
+int sh_add_sphere_wall(sh_ctx *h, const double center[3], double radius, double k, double exponent);
 /* fix gravity --------------------------------------------------------------------------------- */
 int sh_set_gravity(sh_ctx *h, const double g[3]);
 /* neighbor <skin> bin / neigh_modify every N check yes|no ------------------------------------- */

@@ -2,7 +2,7 @@
 
 The class mirrors the LAMMPS input-script surface of the SPHERHARM path (SURVEY §8b):
 set_box / set_quadrature+add_shape (atom_style spherharm) / set_atoms (create_atoms, set quat) /
-pair_coeff (pair_style spherharm) / add_wall / set_gravity / set_neighbor / set_timestep / run.
+pair_coeff (pair_style spherharm) / add_wall / add_cylinder_wall / add_sphere_wall / set_gravity / set_neighbor / set_timestep / run.
 No CPU fallback exists: if the CUDA extension is missing or no device is present, this raises.
 """
 import ctypes as C
@@ -141,6 +141,16 @@ class ShGpu:
     def add_wall(self, point, normal, k, exponent):
         p, nn = _d(point), _d(normal)
         self._ck(self.L.sh_add_wall(self.h, _p(p), _p(nn), C.c_double(k), C.c_double(exponent)))
+
+    def add_cylinder_wall(self, point, axis, radius, k, exponent):
+        """Infinite cylindrical container (particles inside): axis through `point` along `axis`, radius `radius`."""
+        p, u = _d(point), _d(axis)
+        self._ck(self.L.sh_add_cylinder_wall(self.h, _p(p), _p(u), C.c_double(radius), C.c_double(k), C.c_double(exponent)))
+
+    def add_sphere_wall(self, center, radius, k, exponent):
+        """Spherical container (particles inside) of centre `center` and radius `radius`."""
+        c = _d(center)
+        self._ck(self.L.sh_add_sphere_wall(self.h, _p(c), C.c_double(radius), C.c_double(k), C.c_double(exponent)))
 
     def set_gravity(self, g):
         g = _d(g)

@@ -23,6 +23,7 @@
 #include "shape_tables.h"
 #include "step_kernels.cuh"
 #include "atom_stress_kernels.cuh"
+#include "curved_wall_kernels.cuh"
 
 using namespace shgpu;
 
@@ -62,6 +63,7 @@ struct sh_ctx {
   DevBuf<double> d_pk, d_pm, d_pgn, d_pgt, d_pmu, stress_part;
   bool coeff_dirty = true;
   WallSet walls{};
+  CurvedWallSet cwalls{};            // cylinder / sphere containers, applied after the plane walls
   double g[3] = {0, 0, 0}, skin = 0.0, dt = 1e-4, gamma_lin = 0.0, gamma_rot = 0.0;
   int neigh_every = 1, neigh_check = 1;
   // atoms
@@ -176,6 +178,8 @@ AtomView view(sh_ctx *h) {
   return A;
 }
 AtomView view_all(sh_ctx *h) { AtomView A = view(h); A.n = (int)h->n; return A; }
+// plane or curved: the owned atoms' wallf / ewall slots hold this step's wall force and energy
+bool has_walls(const sh_ctx *h) { return h->walls.n > 0 || h->cwalls.n > 0; }
 
 int upload_shapes(sh_ctx *h) {
   if (!h->shapes_dirty) return 0;
@@ -746,12 +750,16 @@ int compute_forces_device(sh_ctx *h) {
     wall_kernel<<<cdiv((int64_t)n * 32, 256), 256, 0, h->stream>>>(A, h->d_shapes.p, h->walls, h->ewall.p);
     h->kernel_launches++;
   }
+  if (h->cwalls.n > 0 && n > 0) {
+    curved_wall_kernel<<<cdiv((int64_t)n * 32, 256), 256, 0, h->stream>>>(A, h->d_shapes.p, h->cwalls, h->ewall.p, h->walls.n > 0);
+    h->kernel_launches++;
+  }
   // newton on: the ghosts have rows too, holding the reactions of the cross-rank pairs evaluated here
   const int nrows = h->list_valid && h->nrows > n ? h->nrows : n;
   if (nrows > 0) {
     AtomView G2 = view_all(h);
     G2.n = nrows;
-    gather_kernel<<<cdiv(nrows, 256), 256, 0, h->stream>>>(G2, h->nbr_off.p, h->slot.p, h->slot_stride, h->walls.n > 0 ? n : 0);
+    gather_kernel<<<cdiv(nrows, 256), 256, 0, h->stream>>>(G2, h->nbr_off.p, h->slot.p, h->slot_stride, has_walls(h) ? n : 0);
     h->kernel_launches++;
   }
   if (newton_dd) { int rc = dd_reverse(h); if (rc) return rc; }
@@ -1077,6 +1085,32 @@ int sh_add_wall(sh_ctx *h, const double point[3], const double normal[3], double
   h->walls.k[w] = k; h->walls.m[w] = exponent;
   h->forces_valid = false;
   return 0;
+}
+
+namespace {
+int add_curved_wall(sh_ctx *h, int type, const double c[3], const double u[3], double radius, double k, double exponent) {
+  if (h->cwalls.n >= SH_MAX_CURVED_WALLS) return fail(h, "too many curved walls");
+  if (!(radius > 0)) return fail(h, "curved wall: need radius > 0");
+  if (!(k >= 0) || !(exponent >= 1.0)) return fail(h, "curved wall: need k >= 0, exponent >= 1");
+  const int w = h->cwalls.n++;
+  h->cwalls.type[w] = type;
+  for (int d = 0; d < 3; d++) { h->cwalls.c[w][d] = c[d]; h->cwalls.u[w][d] = u[d]; }
+  h->cwalls.R[w] = radius; h->cwalls.k[w] = k; h->cwalls.m[w] = exponent;
+  h->forces_valid = false;
+  return 0;
+}
+}  // namespace
+
+int sh_add_cylinder_wall(sh_ctx *h, const double point[3], const double axis[3], double radius, double k, double exponent) {
+  const double nn = std::sqrt(axis[0] * axis[0] + axis[1] * axis[1] + axis[2] * axis[2]);
+  if (!(nn > 0)) return fail(h, "cylinder wall axis is zero");
+  const double u[3] = {axis[0] / nn, axis[1] / nn, axis[2] / nn};
+  return add_curved_wall(h, CWALL_CYLINDER, point, u, radius, k, exponent);
+}
+
+int sh_add_sphere_wall(sh_ctx *h, const double center[3], double radius, double k, double exponent) {
+  const double u[3] = {0, 0, 0};
+  return add_curved_wall(h, CWALL_SPHERE, center, u, radius, k, exponent);
 }
 
 int sh_set_gravity(sh_ctx *h, const double g[3]) { for (int d = 0; d < 3; d++) h->g[d] = g[d]; return 0; }
@@ -1521,7 +1555,7 @@ int sh_get_energy(const sh_ctx *hc, double *ke_trans, double *ke_rot, double *e_
         CU(cudaMemcpy(e.data(), h->pres.p + (size_t)h->pres_stride, h->npairs * sizeof(double), cudaMemcpyDeviceToHost));
         for (double vv : e) ec += vv;
       }
-      if (h->walls.n > 0) {
+      if (has_walls(h)) {
         std::vector<double> e(n);
         CU(cudaMemcpy(e.data(), h->ewall.p, n * sizeof(double), cudaMemcpyDeviceToHost));
         for (double vv : e) ec += vv;
@@ -1596,7 +1630,7 @@ int sh_get_atom_stress(const sh_ctx *hc, int64_t n, int mode, double *virial, do
     S.nbr_off = h->nbr_off.p; S.epair = h->as_epair.p; S.pair_i = h->pair_i.p; S.pair_j = h->pair_j.p; S.pair_img = h->pair_img.p;
     S.pres = h->pres.p; S.pres_stride = h->pres_stride;
     for (int d = 0; d < 3; d++) S.L[d] = h->hi[d] - h->lo[d];
-    S.ewall = h->forces_valid && h->walls.n > 0 ? h->ewall.p : nullptr;
+    S.ewall = h->forces_valid && has_walls(h) ? h->ewall.p : nullptr;
     S.vir = h->as_vir.p; S.kin = h->as_kin.p; S.en = h->as_en.p; S.cnt = h->as_cnt.p; S.ghost_rec = h->as_send.p;
     atom_stress_row_kernel<<<cdiv(nall, 128), 128, 0, h->stream>>>(S);
     h->kernel_launches++;

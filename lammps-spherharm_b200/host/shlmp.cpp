@@ -10,12 +10,17 @@
 // create_box <ntypes> <region> ; create_atoms <type> single x y z ; read_data <file> ; mass/density via
 // `set type <t> density <rho>` ; set atom <id> quat a b c theta | quat/random <seed> ; velocity all set
 // vx vy vz ; velocity <id> set ... ; pair_style spherharm ; pair_coeff i j k exponent [gamma_n gamma_t mu] ; fix <id> <grp>
-// nve/sh | wall/spherharm <xplane|yplane|zplane> <pos> <k> <exponent> [hi] | gravity <g> vector x y z |
-// viscous <gamma> ; neighbor <skin> bin ; neigh_modify every N [check yes|no] ; timestep ; thermo N ;
+// nve/sh | wall/spherharm <xplane|yplane|zplane> <pos> <k> <exponent> [hi] | wall/spherharm zcylinder <radius> <k>
+// <exponent> | wall/spherharm sphere <cx> <cy> <cz> <radius> <k> <exponent> | gravity <g> vector x y z | viscous <gamma> ;
+// neighbor <skin> bin ; neigh_modify every N [check yes|no] ; timestep ; thermo N ;
 // compute <id> all stress/atom NULL [ke] [pair] [virial] [branch center|centroid] | pe/atom | contact/atom ;
 // dump <id> all custom N <file> <columns> (id type x y z vx vy vz qw qx qy qz fx fy fz tqx tqy tqz angmomx angmomy angmomz
 // c_ID c_ID[k]) ; run N ; write_restart <file> ; read_restart <file> ; print "..." ;
 // fix <id> <grp> deform N xy erate <rate> remap v   (Lees-Edwards shear: flow x, gradient y)
+//
+// fix wall/spherharm zcylinder: particles inside an infinite cylinder about the z axis through x = y = 0, as LAMMPS
+// `fix wall/gran ... zcylinder`.  fix wall/spherharm sphere (a shlmp extension): particles inside a sphere.  At most 8
+// curved walls; they use the plane walls' contact law k V^exponent on the volume outside the wall.
 //
 // compute stress/atom gives LAMMPS's 6-vector -(K + W) (xx yy zz xy xz yz; K = m v v, W the per-atom pair virial of
 // sh_get_atom_stress) in stress x volume units.  `branch centroid` (a shlmp extension) takes W from the contact branch
@@ -147,6 +152,8 @@ struct Shlmp {
   std::vector<Coeff> coeffs;
   struct Wall { double p[3], n[3], k, e; };
   std::vector<Wall> walls;
+  struct CWall { bool cyl; double c[3], R, k, e; };   // zcylinder (c = 0) or sphere (c = centre)
+  std::vector<CWall> cwalls;
   double g[3] = {0, 0, 0}, gamma = 0, skin = 0.1, dt = 1e-4;
   int every = 1, check = 1, thermo = 0;
   int64_t step = 0;
@@ -214,6 +221,10 @@ struct Shlmp {
     }
     for (auto &c : coeffs) { ck(sh_pair_coeff(h, c.i - 1, c.j - 1, c.k, c.e)); if (c.gn > 0 || c.gt > 0) ck(sh_pair_dissipation(h, c.i - 1, c.j - 1, c.gn, c.gt, c.mu)); }
     for (auto &w : walls) ck(sh_add_wall(h, w.p, w.n, w.k, w.e));
+    for (auto &w : cwalls) {
+      const double zaxis[3] = {0, 0, 1};
+      ck(w.cyl ? sh_add_cylinder_wall(h, w.c, zaxis, w.R, w.k, w.e) : sh_add_sphere_wall(h, w.c, w.R, w.k, w.e));
+    }
     ck(sh_set_gravity(h, g));
     ck(sh_set_damping(h, gamma, gamma));
     ck(sh_set_neighbor(h, skin, every, check));
@@ -369,7 +380,7 @@ struct Shlmp {
     }
   }
   void run(int64_t nsteps) {
-    if (dry) { init(); if (shear_rate != 0.0 && !(periodic[0] && periodic[1])) error_all(FLERR, "fix deform xy needs a box periodic in x and y"); printf("check: run %lld with %zu atoms, %zu shape(s), %zu wall(s) OK\n", (long long)nsteps, avec.nlocal(), avec.shape_files.size(), walls.size()); step += nsteps; return; }
+    if (dry) { init(); if (shear_rate != 0.0 && !(periodic[0] && periodic[1])) error_all(FLERR, "fix deform xy needs a box periodic in x and y"); printf("check: run %lld with %zu atoms, %zu shape(s), %zu wall(s) OK\n", (long long)nsteps, avec.nlocal(), avec.shape_files.size(), walls.size() + cwalls.size()); step += nsteps; return; }
     if (!nve_defined && master()) fprintf(stderr, "WARNING: no fix nve/sh defined; atoms are integrated by the device step anyway\n");
     init();
     ck(sh_compute_forces(h));
@@ -580,6 +591,18 @@ void execute(Shlmp &S, const std::vector<std::string> &t) {
     const std::string &style = t[3];
     if (style == "nve/sh") { S.nve_defined = true; return; }
     if (style == "wall/spherharm") {
+      need(5);
+      if (t[4] == "zcylinder" || t[4] == "sphere") {
+        const bool cyl = t[4] == "zcylinder";
+        if (t.size() != (cyl ? 8u : 11u)) error_all(FLERR, "Illegal fix wall/spherharm command");
+        Shlmp::CWall w{}; w.cyl = cyl;
+        size_t a = 5;
+        if (!cyl) for (int d = 0; d < 3; d++) w.c[d] = std::stod(t[a++]);
+        w.R = std::stod(t[a]); w.k = std::stod(t[a + 1]); w.e = std::stod(t[a + 2]);
+        if (!(w.R > 0) || !(w.k >= 0) || !(w.e >= 1.0)) error_all(FLERR, "Illegal fix wall/spherharm command");
+        if (S.cwalls.size() >= 8) error_all(FLERR, "Illegal fix wall/spherharm command: at most 8 zcylinder / sphere walls");
+        S.cwalls.push_back(w); return;
+      }
       need(8);
       Shlmp::Wall w{}; const int d = t[4] == "xplane" ? 0 : t[4] == "yplane" ? 1 : t[4] == "zplane" ? 2 : -1;
       if (d < 0) error_all(FLERR, "Illegal fix wall/spherharm command");

@@ -155,6 +155,24 @@ def config2_wall(n_side=10, lmax=20, grid=(32, 64), seed=2, k=1e4, exponent=1.0)
                 walls=[((0, 0, 0), (0, 0, 1), k, exponent)], gravity=(0, 0, -9.81), skin=0.2, dt=2e-4)
 
 
+def config_silo(n_layers=16, radius=6.0, lmax=20, grid=(32, 64), seed=4, k=1e4, exponent=1.0):
+    """Silo filling: mono-shape SH ellipsoids (semi-axes 1, 0.8, 0.6) on a square lattice of spacing 2.2 inside an
+    infinite z-cylinder of the given radius about x = y = 0, settling under gravity onto the floor plane z = 0."""
+    a, b = ellipsoid_shape(lmax)
+    rng = np.random.default_rng(seed)
+    g = np.arange(-radius, radius + 1e-9, 2.2)
+    gx, gy = np.meshgrid(g - g.mean(), g - g.mean(), indexing="ij")
+    disc = np.stack([gx.ravel(), gy.ravel()], 1)
+    disc = disc[np.hypot(disc[:, 0], disc[:, 1]) <= radius - 1.3]
+    pos = np.concatenate([np.column_stack([disc, np.full(len(disc), 1.2 + 2.2 * l)]) for l in range(n_layers)])
+    n = len(pos)
+    return dict(name="silo_%d" % n, lmax=lmax, grid=grid, shapes=[(a, b)], density=1.0,
+                shape_id=np.zeros(n, np.int32), x=pos, v=np.zeros((n, 3)), quat=random_quaternions(rng, n),
+                angmom=np.zeros((n, 3)), box=None, coeff=(k, exponent), walls=[((0, 0, 0), (0, 0, 1), k, exponent)],
+                curved_walls=[("cylinder", (0, 0, 0), (0, 0, 1), radius, k, exponent)], gravity=(0, 0, -9.81),
+                skin=0.2, dt=2e-4)
+
+
 def packing(ncell, lmax, grid, nshapes=8, seed=30, nn_frac=1.9, periodic=True, k=1e3, exponent=1.0,
             vel_sigma=0.05, name="packing", skin=0.05, dt=1e-4):
     """Dense synthetic packing: FCC sites at nn distance nn_frac*Rmax-scale with random orientations and
@@ -235,6 +253,14 @@ def apply(sim, cfg):
                     sim.pair_dissipation(i, j, gn, gt, mu)
     for (pt, nrm, kw, ew) in cfg["walls"]:
         sim.add_wall(pt, nrm, kw, ew)
+    # optional: ("cylinder", point, axis, radius, k, exponent) or ("sphere", centre, radius, k, exponent), in order
+    for wall in cfg.get("curved_walls", ()):
+        if wall[0] == "cylinder":
+            sim.add_cylinder_wall(*wall[1:])
+        elif wall[0] == "sphere":
+            sim.add_sphere_wall(*wall[1:])
+        else:
+            raise ValueError("unknown curved wall %r" % (wall[0],))
     sim.set_gravity(cfg["gravity"])
     sim.set_neighbor(cfg["skin"], 1, 1)
     sim.set_timestep(cfg["dt"])

@@ -49,6 +49,9 @@ def main(outdir=os.path.join(ROOT, "examples")):
     # BASELINE configs[3] at example size: periodic mono-shape packing sheared by Lees-Edwards images (in.shear_box)
     cfg = W.shear_box(W.packing((5, 4, 4), 20, (32, 64), nshapes=1, seed=33, periodic=True, vel_sigma=0.3), 0.6)
     write_data(os.path.join(outdir, "data.shear_320"), cfg, (cfg["box"][0], cfg["box"][1]))
+    # silo filling (in.silo): particles inside a z-cylinder of radius 6 above a floor plane at z = 0
+    cfg = W.config_silo()
+    write_data(os.path.join(outdir, "data.silo_256"), cfg, ((-7.0, -7.0, 0.0), (7.0, 7.0, cfg["x"][:, 2].max() + 3.0)))
 
 
 if __name__ == "__main__":
